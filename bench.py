@@ -21,6 +21,10 @@ the same scene on one GPU ("mgpu_parity").
                with slope + intercept
 
   python bench.py --gpus N --steps K --warmup W [--impl reference] [--poses P --voxels M --precision fp64|tensor]
+                  [--dump-outputs DIR]
+
+--dump-outputs DIR writes what the last timed step returned as DIR/<name>.npy (float64). The inputs depend on the
+arguments only, so two builds run with the same arguments can be compared output for output.
 """
 import argparse
 import json
@@ -34,11 +38,24 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True  # the source tree may be read-only; the benchmark leaves nothing in it
 
 PTS = 40
 NOISE = 0.01
 RANGE = 2.0
 SEED = 10
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir, arrays):
+    """Writes every array of `arrays` as out_dir/<name>.npy in float64."""
+    arrays = {k: np.asarray(v, dtype=np.float64) for k, v in arrays.items()}
+    total = sum(a.nbytes for a in arrays.values())
+    if total > DUMP_LIMIT_BYTES:
+        raise ValueError(f"--dump-outputs: {total} bytes exceed the {DUMP_LIMIT_BYTES} byte limit")
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
 
 
 def peaks():
@@ -217,14 +234,15 @@ class CpuArm:
             o.residual(self.init)                                   # evaluate_only_residual, 1 thread
             tr.append(time.perf_counter() - t0)
         t0 = time.perf_counter()
-        self.big.lm_step(H, g, 0.01, self.init)                     # (H + uD).ldlt().solve(-g) + update, 1 thread
+        dx, trial, _ = self.big.lm_step(H, g, 0.01, self.init)      # (H + uD).ldlt().solve(-g) + update, 1 thread
         t_solve = time.perf_counter() - t0
+        self.last = {"H": H, "g": g, "r": r, "dx": dx, "poses_trial": trial}   # of the larger sample
         dm = float(self.m2 - self.m1)
         se, sr = (te[1] - te[0]) / dm, (tr[1] - tr[0]) / dm          # seconds per voxel
         ie, ir = te[0] - se * self.m1, tr[0] - sr * self.m1          # per-evaluation O(n^2) overhead
-        if ie < 0:   # timing noise made the small sample look super-linear: fall back to the proportional estimate
+        if ie < 0 or se <= 0:   # timing noise made the samples look super- or sub-linear: the proportional estimate
             se, ie = te[1] / self.m2, 0.0
-        if ir < 0:
+        if ir < 0 or sr <= 0:
             sr, ir = tr[1] / self.m2, 0.0
         t_iter = (ie + se * voxels_total) + (ir + sr * voxels_total) + t_solve
         detail = {"t_eval_s": te, "t_residual_s": tr, "t_solve_s": t_solve, "eval_s_per_voxel": se,
@@ -252,7 +270,7 @@ def ref_headers_check(n_poses, m_small, port_eval_s):
             "t0 = time.perf_counter(); prob.divide_thread_left(init)\n"
             "print(json.dumps({'t': time.perf_counter() - t0}))\n") % (ROOT, n_poses, m_small, n_poses)
     try:
-        out = subprocess.run([sys.executable, "-c", code], capture_output=True, text=True, timeout=300)
+        out = subprocess.run([sys.executable, "-B", "-c", code], capture_output=True, text=True, timeout=300)
         res = json.loads(out.stdout.strip().splitlines()[-1])
         if res is None:
             return None
@@ -303,6 +321,11 @@ def run_reference(args, rank, world):
             its.append(t)
     t_iter = float(np.mean(its))
     val = 1.0 / t_iter
+    if args.dump_outputs:
+        out = dict(arm.last)
+        H = out.pop("H")
+        rows = np.sort(np.random.default_rng(SEED).choice(len(H), min(len(H), 64), replace=False))
+        dump_outputs(args.dump_outputs, dict(out, H_rows=H[rows], H_row_index=rows))   # 64 seeded rows of the n x n H
     chk = ref_headers_check(n, args.cpu_sample_small, detail["t_eval_s"][0])  # once, outside the timed steps
     line = {
         "impl": "reference", "metric": "ba_iterations_per_sec", "value": val, "unit": "iter/s", "n_gpus": args.gpus,
@@ -370,7 +393,11 @@ def main():
     ap.add_argument("--cpu-sample-large", type=int, default=1024)
     ap.add_argument("--no-cpu", action="store_true")
     ap.add_argument("--no-e2e", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed step returned as DIR/<name>.npy (float64, at most 64 MB)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.warmup < 3:
         args.warmup = 3
 
@@ -435,6 +462,12 @@ def main():
     barrier()
     clocks = sampler.stop(mark)
     tm = ctx.timings()
+    assert len(trace) == args.steps, (len(trace), args.steps)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, {
+            "poses": poses,   # N x 12 after the last timed step
+            "lm_trace": [[t_[k_] for k_ in ("r1", "r2", "u", "v", "q", "q1", "accepted", "recomputed_hess", "not_pd")]
+                         for t_ in trace]})
     t = torch.tensor([ms], dtype=torch.float64, device="cuda")
     if world > 1:
         dist.all_reduce(t, op=dist.ReduceOp.MAX)

@@ -1,8 +1,8 @@
 """The CUDA path against the REFERENCE'S OWN CODE, on the GPU box.
 
-oracle/_ref/libbalm_ref.so -- /root/reference/src/benchmark/bavoxel.hpp + include/tools.hpp compiled where they lie behind
-oracle/ref_harness.cpp (stand-ins for the absent Eigen / PCL / ROS headers, oracle/ref_stubs) -- is built in the container
-that holds /root/reference and travels with the snapshot. Here the library's results (through the C ABI) are compared with
+oracle/_ref/libbalm_ref.so -- the reference's src/benchmark/bavoxel.hpp + include/tools.hpp compiled where they lie behind
+oracle/ref_harness.cpp (stand-ins for the absent Eigen / PCL / ROS headers, oracle/ref_stubs) -- is built where
+BALM_REFERENCE_DIR names a checkout of the reference (tests/test_gpu_vs_restatement.py runs the same inputs elsewhere). Here the library's results (through the C ABI) are compared with
 what the reference's own VOX_HESS / BALM2 / OCTO_TREE_ROOT produce on the same inputs: no restatement in between.
 Tolerances as in tests/test_gpu_parity.py (SURVEY.md 8d)."""
 import numpy as np
@@ -14,7 +14,7 @@ from oracle import oracle_py as orc
 from oracle import ref_py as ref
 
 pytestmark = [pytest.mark.gpu,
-              pytest.mark.skipif(not ref.available(), reason="oracle/_ref/libbalm_ref.so did not travel (built where /root/reference exists)")]
+              pytest.mark.skipif(not ref.available(), reason="oracle/_ref/libbalm_ref.so not built (needs BALM_REFERENCE_DIR)")]
 
 PRECS = [pytest.param(0, id="fp64"), pytest.param(1, id="tensor")]
 TOLH = {0: 1e-9, 1: 1e-8}

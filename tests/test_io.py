@@ -71,9 +71,12 @@ def test_pose_packing_and_rsme():
     assert abs(rot - np.linalg.norm(w)) < 1e-9 and abs(tran - 0.1 * np.sqrt(3)) < 1e-12
 
 
-@pytest.mark.skipif(not os.path.isdir("/root/reference/datas/benchmark_realworld"), reason="reference dataset not here")
+REALWORLD = os.path.join(os.environ.get("BALM_REFERENCE_DIR", "/nonexistent"), "datas", "benchmark_realworld")
+
+
+@pytest.mark.skipif(not os.path.isdir(REALWORLD), reason="BALM_REFERENCE_DIR does not name a checkout with the dataset")
 def test_reads_the_reference_dataset():
-    d = "/root/reference/datas/benchmark_realworld"
+    d = REALWORLD
     R, p, t = io.read_pose_csv(os.path.join(d, "alidarPose.csv"))
     assert len(R) == 177 and np.allclose(np.einsum("nij,nkj->nik", R, R), np.eye(3), atol=1e-5)  # the csv stores six decimals
     xyz = io.read_pcd(os.path.join(d, "full0.pcd"))

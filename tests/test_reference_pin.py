@@ -1,6 +1,6 @@
 """The restated oracles against the REFERENCE'S OWN CODE.
 
-oracle/_ref/libbalm_ref.so is /root/reference/src/benchmark/bavoxel.hpp + /root/reference/include/tools.hpp compiled where
+oracle/_ref/libbalm_ref.so is the reference's src/benchmark/bavoxel.hpp + include/tools.hpp ($BALM_REFERENCE_DIR) compiled where
 they lie (oracle/Makefile, oracle/ref_harness.cpp) against stand-ins for the absent Eigen / PCL / ROS headers
 (oracle/ref_stubs: generic dense arithmetic, nothing of the reference). These tests pin
   oracle/balm_oracle.c       against  VOX_HESS::{push_voxel, left_evaluate_acc2, evaluate_only_residual},
@@ -19,7 +19,7 @@ import scenes
 from oracle import oracle_py as orc
 from oracle import ref_py as ref
 
-pytestmark = pytest.mark.skipif(not ref.available(), reason="oracle/_ref/libbalm_ref.so not built (needs /root/reference)")
+pytestmark = pytest.mark.skipif(not ref.available(), reason="oracle/_ref/libbalm_ref.so not built (needs BALM_REFERENCE_DIR)")
 
 
 def _pose_err(a, b):
@@ -193,10 +193,10 @@ def test_repeated_marginalisation_matches_the_reference_octree():
         win -= mg
 
 
-REALWORLD = "/root/reference/datas/benchmark_realworld"
+REALWORLD = os.path.join(os.environ.get("BALM_REFERENCE_DIR", "/nonexistent"), "datas", "benchmark_realworld")
 
 
-@pytest.mark.skipif(not os.path.exists(os.path.join(REALWORLD, "alidarPose.csv")), reason="the reference's dataset is not on this box")
+@pytest.mark.skipif(not os.path.exists(os.path.join(REALWORLD, "alidarPose.csv")), reason="BALM_REFERENCE_DIR does not name a checkout with the dataset")
 def test_association_restatement_matches_the_reference_octree_on_its_own_dataset():
     """The first 16 scans of datas/benchmark_realworld (every 4th point), re-anchored to pose 0 and cut with the constants
     of benchmark_realworld.cpp:163-185 (voxel_size 2, eigen ratios {1/16, 1/16, 1/9} stored as float): real lidar data has
@@ -237,6 +237,43 @@ def test_golden_fixtures_are_outputs_of_the_reference_code(fixture):
     assert rot <= 1e-10 and tra <= 1e-10, (rot, tra)
 
 
+def test_restatement_fixture_is_output_of_the_reference_code():
+    """tests/golden/restatement_outputs.npz (what tests/test_gpu_vs_restatement.py holds the GPU to) was written with the
+    oracle and tests/assoc_ref.py. The reference's own VOX_HESS / BALM2 / octree on the same inputs give the same values."""
+    import restated_cases as rc
+    d = rc.load()
+    for k, (n_poses, n_planes, drop, with_fix) in enumerate(rc.EVAL_SCENES):
+        sc = rc.eval_scene(n_poses, n_planes, drop, with_fix)
+        p = ref.Problem(n_poses, sc["row_ptr"], sc["pose_idx"], sc["obs10"], sc["fix10"])
+        assert p.pushed() == n_planes and np.array_equal(p.coeffs(), rc.coe_of(sc))
+        for name in ("poses_init", "poses_gt"):
+            H, g, r = p.divide_thread_left(sc[name])
+            assert abs(r - float(d[f"eval{k}_{name}_r"])) <= 1e-11 * abs(r)
+            assert np.abs(g - d[f"eval{k}_{name}_g"]).max() <= 1e-10 * np.abs(g).max()
+            assert np.abs(np.diag(H) - d[f"eval{k}_{name}_Hdiag"]).max() <= 1e-10 * np.abs(np.diag(H)).max()
+            assert rc.probes_close(H, d[f"eval{k}_{name}_Hprobes"], 1e-10)
+            assert abs(p.evaluate_only_residual(sc[name]) - float(d[f"eval{k}_{name}_residual"])) <= 1e-11 * abs(r)
+        H, g, r = p.left_evaluate_acc2(sc["poses_init"], *rc.eval_range(n_planes))
+        assert abs(r - float(d[f"eval{k}_range_r"])) <= 1e-11 * abs(r)
+        assert rc.probes_close(H, d[f"eval{k}_range_Hprobes"], 1e-10)
+    sc = rc.lm_scene()
+    p = ref.Problem(24, sc["row_ptr"], sc["pose_idx"], sc["obs10"])
+    rot, tra = _pose_err(p.damping_iter(sc["poses_init"]), d["lm_poses"])
+    assert rot <= 1e-8 and tra <= 1e-8, (rot, tra)
+    n, mg, kw = rc.ASSOC_N, rc.ASSOC_MG, rc.ASSOC_KW
+    pts, frs, poses, poses12, opt = rc.assoc_inputs()
+    s = _session_from_scans(pts.astype(np.float32), frs, poses12, n, **kw)
+    keys, rp, pi, ob, fx, co, lay = s.export(n, with_layers=True)
+    assert np.array_equal(keys, d["assoc_keys"]) and np.array_equal(lay, d["assoc_layers"])
+    assert np.array_equal(rp, d["assoc_row_ptr"]) and np.array_equal(pi, d["assoc_pose_idx"])
+    assert np.array_equal(co, d["assoc_coe"]) and rc.probes_close(ob, d["assoc_obs_probes"], 1e-11)
+    s.marginalize(mg, opt, n)
+    keys1, rp1, pi1, ob1, fx1, co1 = s.export(n - mg)
+    assert np.array_equal(keys1, d["marg_keys"]) and np.array_equal(rp1, d["marg_row_ptr"])
+    assert np.array_equal(pi1, d["marg_pose_idx"]) and np.array_equal(co1, d["marg_coe"])
+    assert rc.probes_close(ob1, d["marg_obs_probes"], 1e-11) and rc.probes_close(fx1, d["marg_fix_probes"], 1e-12)
+
+
 @pytest.mark.parametrize("n_poses,n_planes,drop,with_fix", [(6, 40, 0.0, False), (9, 60, 0.4, True)])
 def test_right_update_restatement_matches_the_reference(n_poses, n_planes, drop, with_fix):
     """tests/numpy_acc2.py (the second reference-side pin of residual and gradient, used on the oracle and on the GPU path)
@@ -253,7 +290,7 @@ def test_right_update_restatement_matches_the_reference(n_poses, n_planes, drop,
 
 
 # ---------------- the consistency experiment (src/simulation/BAs_left.hpp, toolss.hpp) ----------------
-sim = pytest.mark.skipif(not ref.sim_available(), reason="oracle/_ref/libbalm_ref_sim.so not built (needs /root/reference)")
+sim = pytest.mark.skipif(not ref.sim_available(), reason="oracle/_ref/libbalm_ref_sim.so not built (needs BALM_REFERENCE_DIR)")
 
 
 @sim

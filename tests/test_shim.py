@@ -59,7 +59,7 @@ def test_shim_runs_reference_call_pattern(prec):
 
 
 # ---- the shim on top of the REFERENCE'S OWN tools.hpp (PointCluster, IMUST; stand-in Eigen / PCL of oracle/ref_stubs) ----
-REF_INC = "/root/reference/include"
+REF_INC = os.path.join(os.environ.get("BALM_REFERENCE_DIR", "/nonexistent"), "include")
 EXE3 = os.path.join(ROOT, "tests", "shim_reference_types.bin")
 
 
@@ -71,7 +71,7 @@ def build_reference_types():
                            "-Wl,-rpath," + lib, "-ldl", "-lpthread", "-lrt"])
 
 
-@pytest.mark.skipif(not os.path.exists(os.path.join(REF_INC, "tools.hpp")), reason="/root/reference is not on this box")
+@pytest.mark.skipif(not os.path.exists(os.path.join(REF_INC, "tools.hpp")), reason="BALM_REFERENCE_DIR does not name a checkout of the reference")
 def test_shim_compiles_on_the_reference_types():
     """#include "tools.hpp" (the reference's, verbatim) + the shim in BALM_B200_WITH_EIGEN mode with its default plptrs type
     pcl::PointCloud<PointType>::Ptr: what a BALM translation unit looks like after swapping bavoxel.hpp for the shim."""
@@ -85,7 +85,7 @@ def test_shim_runs_on_the_reference_types(prec):
     if os.path.exists(os.path.join(REF_INC, "tools.hpp")):
         build_reference_types()
     if not os.path.exists(EXE3):
-        pytest.skip("tests/shim_reference_types.bin was not built (needs /root/reference at build time)")
+        pytest.skip("tests/shim_reference_types.bin was not built (needs BALM_REFERENCE_DIR at build time)")
     out = subprocess.run([EXE3, str(prec)], capture_output=True, text=True, timeout=120)
     assert out.returncode == 0, out.stdout + out.stderr
     assert "shim_reference_types: residual" in out.stdout
